@@ -18,6 +18,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -49,7 +50,27 @@ def parse_args():
     ap.add_argument("--no-l2-flush", action="store_true")
     ap.add_argument("--worker-threads", type=int, default=6,
                     help="threads (= Nets = streams) of the Worker the pipelined e2e leg serves requests with; 0 skips it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<output name>.npy (inputs are seeded: two "
+                         "builds run with the same arguments can be compared output for output)")
     return ap.parse_args()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """{name: array} -> dirname/<name>.npy in float32 (float64 kept). Past DUMP_LIMIT_BYTES in all, every array is cut to
+    the same share of its rows (images), chosen with a fixed seed, so that two runs still write the same rows."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a if a.dtype == np.float64 else a.astype(np.float32) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            rows = max(1, a.shape[0] * DUMP_LIMIT_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def peaks():
@@ -153,11 +174,12 @@ def cpu_oracle_images_per_s(model, precision, batch, budget_s=20.0, steps=None, 
         t0 = time.perf_counter()
         run()
         steps = int(min(200, max(3, budget_s / 4.0 / max(time.perf_counter() - t0, 1e-4))))
+    out = None
     t0 = time.perf_counter()
     for _ in range(steps):
-        run()
+        out = run()
     dt = time.perf_counter() - t0
-    return {"value": n_img * steps / dt, "unit": "images/s", "cores": O.num_threads(), "kind": "port",
+    return {"value": n_img * steps / dt, "unit": "images/s", "cores": O.num_threads(), "kind": "port", "outputs": out,
             "sample": "%d step(s) x %d image(s) of %s %s via oracle/model_walker.py (x86-semantics restatement, %s"
                       "OpenMP, not Anakin's MKL/xbyak build)" % (steps, n_img, model, precision,
                                                                   "AVX-512 VNNI convolutions on weights packed once, AVX-512 pooling, " if vnni else
@@ -237,6 +259,8 @@ def run_reference(args):
     if rank != 0:
         return
     r = cpu_oracle_images_per_s(args.model, args.precision, args.batch, steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["outputs"])
     line = {"impl": "reference", "metric": "%s %s images/sec" % (MODEL_NAMES.get(args.model, args.model), args.precision.upper()),
             "value": r["value"], "unit": "images/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -352,6 +376,9 @@ def main():
             stops[i].record(stream)
     barrier()
     t_region1 = time.perf_counter()
+    if args.dump_outputs:
+        suffix = "_rank%d" % rank if world > 1 else ""
+        dump_outputs(args.dump_outputs, {name + suffix: net.get_output(name) for name in net.out_names})
     per_step = np.array([s.elapsed_time(e) for s, e in zip(starts, stops)])
     total_ms = float(per_step.sum())
     clocks_window = "timed region"
@@ -412,10 +439,9 @@ def main():
     sampler2 = ClockSampler(local_rank, period_ms=1000)
     if rank == 0 and T > 0 and not os.environ.get("BENCH_NO_SAMPLER_E2E"):
         sampler2.start()
+    tmpdir = tempfile.TemporaryDirectory(prefix="bench_")    # the source tree may be read-only
     if T > 0:
-        tmpdir = os.path.join(ROOT, ".bench_tmp")
-        os.makedirs(tmpdir, exist_ok=True)
-        mpath = os.path.join(tmpdir, "model_rank%d.anakin.bin" % rank)
+        mpath = os.path.join(tmpdir.name, "model_rank%d.anakin.bin" % rank)
         with open(mpath, "wb") as f:
             f.write(blob)
         W = api.Worker(mpath, prec, threads=T, devices=[local_rank], batch=batch)

@@ -1,65 +1,105 @@
-"""CPU suite (-m "not gpu"): pins the oracle restatement to the reference's own naive test oracle
-(oracle/_ref, compiled from /root/reference -- skipped where that tree is absent) and to the
-committed golden fixtures; property tests of the oracle itself."""
+"""CPU suite (-m "not gpu"): pins the oracle restatement to what the reference's own code returned (its naive test
+oracles, shape rules, BN fold, quantisation helpers and x86 INT8 convolution, compiled into oracle/_ref by
+`make -C oracle ref`; their results are stored in tests/golden/reference_oracle.json) and to the committed golden
+fixtures; property tests of the oracle itself."""
+import hashlib
+import json
 import os
 
 import numpy as np
 import pytest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# What the reference returned for every case below, so that the comparison runs without the reference's sources: a
+# SHA-256 digest per output array (the arrays themselves come to megabytes) and plain JSON for scalars and shapes.
+# `B200_RECORD_REFERENCE=1 pytest tests/test_cpu_oracle.py`, with oracle/_ref built, re-runs the reference on the same
+# seeded inputs and rewrites the stored results.
+REF_GOLD = os.path.join(GOLD, "reference_oracle.json")
 
 
-def _need_ref(oracle):
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not built (no /root/reference on this machine)")
+def _digest(a):
+    """dtype, shape and SHA-256 of an array; -0.0 counts as 0.0 and all NaNs as one, as in assert_array_equal."""
+    a = np.ascontiguousarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a).astype(a.dtype) + a.dtype.type(0)
+    return "%s%s %s" % (a.dtype.str, list(a.shape), hashlib.sha256(a.tobytes()).hexdigest())
+
+
+class _Reference:
+    def __init__(self, stored, record):
+        self.stored, self.record, self.new = stored, record, {}
+
+    def value(self, key, run):
+        """The reference's result for case `key`: run() when recording, the stored result otherwise."""
+        if self.record:
+            self.new[key] = json.loads(json.dumps(run()))
+            return self.new[key]
+        assert key in self.stored, "no stored reference result for %r (re-record %s)" % (key, REF_GOLD)
+        return self.stored[key]
+
+    def assert_equal(self, key, got, run):
+        """`got` is bit for bit the array the reference returned for case `key` (run() when recording)."""
+        assert _digest(got) == self.value(key, lambda: _digest(run())), "differs from the reference: %r" % key
+
+
+@pytest.fixture(scope="module")
+def reference(oracle):
+    record = os.environ.get("B200_RECORD_REFERENCE") == "1"
+    if record and oracle.ref_lib() is None:
+        raise RuntimeError("B200_RECORD_REFERENCE=1 needs oracle/_ref (make -C oracle ref)")
+    with open(REF_GOLD) as f:
+        stored = json.load(f)
+    ref = _Reference(stored, record)
+    yield ref
+    if record:
+        stored.update(ref.new)
+        with open(REF_GOLD, "w") as f:       # one case per line
+            f.write("{\n%s\n}\n" % ",\n".join("%s: %s" % (json.dumps(k), json.dumps(v)) for k, v in sorted(stored.items())))
 
 
 # shape sweep of reference test/saber/test_saber_conv.cpp:886-901,1000-1015
 @pytest.mark.parametrize("k,pad,stride,dil", [(1, 0, 1, 1), (3, 1, 1, 1), (3, 1, 2, 1), (3, 0, 1, 2), (3, 1, 2, 2)])
 @pytest.mark.parametrize("cin,cout,hw,n", [(4, 4, 12, 1), (8, 32, 21, 3), (16, 8, 24, 1)])
 @pytest.mark.parametrize("bias,relu", [(True, True), (False, False)])
-def test_conv_f32_matches_reference_oracle(oracle, k, pad, stride, dil, cin, cout, hw, n, bias, relu):
-    _need_ref(oracle)
+def test_conv_f32_matches_reference_oracle(oracle, reference, k, pad, stride, dil, cin, cout, hw, n, bias, relu):
     rng = np.random.default_rng(k * 100 + cin)
     x = rng.uniform(-5, 5, (n, cin, hw, hw)).astype(np.float32)
     w = rng.uniform(-1, 1, (cout, cin, k, k)).astype(np.float32)
     b = rng.uniform(-1, 1, cout).astype(np.float32) if bias else None
     kw = dict(stride=(stride, stride), pad=(pad, pad), dil=(dil, dil), relu=relu)
     a = oracle.conv_f32_nchw(x, w, b, **kw)
-    r = oracle.ref_conv_f32_nchw(x, w, b, **kw)
-    np.testing.assert_array_equal(a, r)
+    reference.assert_equal("conv_f32%r" % ((k, pad, stride, dil, cin, cout, hw, n, bias, relu),), a,
+                           lambda: oracle.ref_conv_f32_nchw(x, w, b, **kw))
     # the vectorised NHWC variant only re-associates the dot product
     fast = oracle.conv_f32_nhwc(np.transpose(x, (0, 2, 3, 1)), w, b, **kw)
     mr, md = oracle.tensor_cmp(np.transpose(a, (0, 2, 3, 1)), fast)
     assert md <= 1e-5 * max(1.0, float(np.abs(a).max())), (mr, md)
 
 
-def test_conv_f32_real_model_shape(oracle):
+def test_conv_f32_real_model_shape(oracle, reference):
     """test_saber_conv.cpp:868-883: 1x3x224x224 -> 64, 3x3, pad 1, bias + relu."""
-    _need_ref(oracle)
     rng = np.random.default_rng(0)
     x = rng.uniform(-5, 5, (1, 3, 224, 224)).astype(np.float32)
     w = rng.uniform(-1, 1, (64, 3, 3, 3)).astype(np.float32)
     b = rng.uniform(-1, 1, 64).astype(np.float32)
-    np.testing.assert_array_equal(oracle.conv_f32_nchw(x, w, b, pad=(1, 1), relu=True),
-                                  oracle.ref_conv_f32_nchw(x, w, b, pad=(1, 1), relu=True))
+    reference.assert_equal("conv_f32 1x3x224x224 -> 64", oracle.conv_f32_nchw(x, w, b, pad=(1, 1), relu=True),
+                           lambda: oracle.ref_conv_f32_nchw(x, w, b, pad=(1, 1), relu=True))
 
 
-def test_conv_f32_groups_beta_alpha(oracle):
-    _need_ref(oracle)
+def test_conv_f32_groups_beta_alpha(oracle, reference):
     rng = np.random.default_rng(1)
     x = rng.uniform(-2, 2, (2, 8, 9, 9)).astype(np.float32)
     w = rng.uniform(-1, 1, (8, 2, 3, 3)).astype(np.float32)
     dst = rng.uniform(-1, 1, (2, 8, 9, 9)).astype(np.float32)
     kw = dict(group=4, pad=(1, 1), beta=0.5, alpha=1.5, dst=dst)
-    np.testing.assert_array_equal(oracle.conv_f32_nchw(x, w, None, **kw), oracle.ref_conv_f32_nchw(x, w, None, **kw))
+    reference.assert_equal("conv_f32 groups beta alpha", oracle.conv_f32_nchw(x, w, None, **kw),
+                           lambda: oracle.ref_conv_f32_nchw(x, w, None, **kw))
 
 
 @pytest.mark.parametrize("unsigned", [False, True])
 @pytest.mark.parametrize("k,pad,stride", [(1, 0, 1), (3, 1, 1), (3, 1, 2)])
 @pytest.mark.parametrize("elt,relu,down", [(False, True, False), (True, True, False), (True, False, True)])
-def test_conv_int8_basic_matches_reference_oracle(oracle, unsigned, k, pad, stride, elt, relu, down):
-    _need_ref(oracle)
+def test_conv_int8_basic_matches_reference_oracle(oracle, reference, unsigned, k, pad, stride, elt, relu, down):
     rng = np.random.default_rng(7 + k + stride)
     x = (rng.integers(0, 256, (2, 10, 10, 8)).astype(np.uint8) if unsigned
          else rng.integers(-128, 128, (2, 10, 10, 8)).astype(np.int8))
@@ -71,43 +111,41 @@ def test_conv_int8_basic_matches_reference_oracle(oracle, unsigned, k, pad, stri
     kw = dict(pad=(pad, pad), stride=(stride, stride), relu=relu, has_elt_sum=elt, sum_scale=0.7, dst=dst,
               round_down=down)
     a = oracle.conv_s8_nhwc_basic(x, w, b, sc, **kw)
-    r = oracle.conv_s8_nhwc_basic(x, w, b, sc, use_ref=True, **kw)
-    np.testing.assert_array_equal(a, r)
+    reference.assert_equal("conv_int8_basic%r" % ((unsigned, k, pad, stride, elt, relu, down),), a,
+                           lambda: oracle.conv_s8_nhwc_basic(x, w, b, sc, use_ref=True, **kw))
 
 
-def test_x86_semantics_agree_with_reference_oracle_on_shared_subset(oracle):
+def test_x86_semantics_agree_with_reference_oracle_on_shared_subset(oracle, reference):
     """The x86-JIT restatement and conv_basic_check_int8 coincide when the bias is integral, the
     output is s8 and there is no residual -- pins oracle_conv_s8_nhwc_x86 to the reference."""
-    _need_ref(oracle)
     rng = np.random.default_rng(11)
     x = rng.integers(-128, 128, (2, 9, 9, 16)).astype(np.int8)
     w = rng.integers(-127, 128, (32, 16, 3, 3)).astype(np.int8)
     b = rng.integers(-1000, 1000, 32).astype(np.int32)
     sc = rng.uniform(0.0005, 0.005, 32).astype(np.float32)
     for relu in (False, True):
-        r = oracle.conv_s8_nhwc_basic(x, w, b, sc, pad=(1, 1), relu=relu, use_ref=True)
         j = oracle.conv_s8_nhwc_x86(x, w, b.astype(np.float32), sc, pad=(1, 1), relu=relu, out_dtype=oracle.DT_INT8)
-        np.testing.assert_array_equal(j, r)
+        reference.assert_equal("conv_int8_basic shared subset relu=%r" % relu, j,
+                               lambda: oracle.conv_s8_nhwc_basic(x, w, b, sc, pad=(1, 1), relu=relu, use_ref=True))
 
 
 @pytest.mark.parametrize("ptype", [1, 2, 3])
 @pytest.mark.parametrize("unsigned", [False, True])
-def test_pool_int8_matches_reference_oracle(oracle, ptype, unsigned):
-    _need_ref(oracle)
+def test_pool_int8_matches_reference_oracle(oracle, reference, ptype, unsigned):
     rng = np.random.default_rng(3)
     x = (rng.integers(0, 128, (2, 13, 13, 8)).astype(np.uint8) if unsigned
          else rng.integers(0, 128, (2, 13, 13, 8)).astype(np.int8))
     a = oracle.pool_s8_nhwc(x, (3, 3), (1, 1), (2, 2), ptype)
-    r = oracle.pool_s8_nhwc(x, (3, 3), (1, 1), (2, 2), ptype, use_ref=True)
-    np.testing.assert_array_equal(a, r)
+    reference.assert_equal("pool_int8%r" % ((ptype, unsigned),), a,
+                           lambda: oracle.pool_s8_nhwc(x, (3, 3), (1, 1), (2, 2), ptype, use_ref=True))
 
 
-def test_tensor_cmp_matches_reference(oracle):
-    _need_ref(oracle)
+def test_tensor_cmp_matches_reference(oracle, reference):
     rng = np.random.default_rng(5)
     a = rng.uniform(-3, 3, 1000).astype(np.float32)
     b = a + rng.uniform(-1e-3, 1e-3, 1000).astype(np.float32)
-    assert oracle.tensor_cmp(a, b) == pytest.approx(oracle.tensor_cmp(a, b, use_ref=True), rel=1e-12)
+    want = reference.value("tensor_cmp", lambda: oracle.tensor_cmp(a, b, use_ref=True))
+    assert oracle.tensor_cmp(a, b) == pytest.approx(tuple(want), rel=1e-12)
 
 
 def test_pool_shape_rule(oracle):
@@ -121,43 +159,42 @@ def test_pool_shape_rule(oracle):
     assert oracle.pool_out_size(7, 7, 7, 7, 0, 0, 1, 1, global_pooling=True) == (1, 1)
 
 
-def test_pool_shape_rule_matches_reference_compute_output_shape(oracle):
+def test_pool_shape_rule_matches_reference_compute_output_shape(oracle, reference):
     """Exhaustive sweep of the restated rule -- and of the product's host-side b200_pool_out_hw -- against the
     reference's own Pooling::compute_output_shape compiled from saber/funcs/pooling.h (oracle/_ref)."""
     import ctypes as C
-    if oracle.ref_pool_out_size(8, 8, 2, 2, 0, 0, 2, 2) is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     from anakin_b200 import saber_abi as A
     lib = A.load()
-    n = 0
-    for h, w in [(7, 7), (12, 13), (14, 14), (21, 24), (56, 56), (112, 112), (224, 224)]:
-        for win in (1, 2, 3, 5, 7):
-            for pad in (0, 1, 2, 3):
-                for stride in (1, 2, 3):
-                    for floor in (False, True):
-                        if win > h + 2 * pad or pad >= win:
-                            continue
-                        want = oracle.ref_pool_out_size(h, w, win, win, pad, pad, stride, stride, False, floor)
-                        assert oracle.pool_out_size(h, w, win, win, pad, pad, stride, stride, False, floor) == want, \
-                            (h, w, win, pad, stride, floor)
-                        d = A.PoolDesc()
-                        d.dtype, d.type, d.n, d.h, d.w, d.c = A.FLOAT, 1, 1, h, w, 16
-                        d.window_h = d.window_w = win
-                        d.pad_h = d.pad_w = pad
-                        d.stride_h = d.stride_w = stride
-                        d.global_pooling, d.floor_as_conv = 0, int(floor)
-                        oh, ow = C.c_int32(), C.c_int32()
-                        assert lib.b200_pool_out_hw(C.byref(d), C.byref(oh), C.byref(ow)) == A.SUCCESS
-                        assert (oh.value, ow.value) == want, (h, w, win, pad, stride, floor)
-                        n += 1
-        assert oracle.pool_out_size(h, w, 3, 3, 0, 0, 1, 1, True) == oracle.ref_pool_out_size(h, w, 3, 3, 0, 0, 1, 1, True)
-    assert n > 500
+    sizes = [(7, 7), (12, 13), (14, 14), (21, 24), (56, 56), (112, 112), (224, 224)]
+    cases = [(h, w, win, pad, stride, floor) for h, w in sizes for win in (1, 2, 3, 5, 7) for pad in (0, 1, 2, 3)
+             for stride in (1, 2, 3) for floor in (False, True) if not (win > h + 2 * pad or pad >= win)]
+    wants = reference.value("pool_out_size sweep", lambda: [
+        oracle.ref_pool_out_size(h, w, win, win, pad, pad, stride, stride, False, floor)
+        for h, w, win, pad, stride, floor in cases])
+    assert len(wants) == len(cases) > 500
+    for (h, w, win, pad, stride, floor), want in zip(cases, wants):
+        want = tuple(want)
+        assert oracle.pool_out_size(h, w, win, win, pad, pad, stride, stride, False, floor) == want, \
+            (h, w, win, pad, stride, floor)
+        d = A.PoolDesc()
+        d.dtype, d.type, d.n, d.h, d.w, d.c = A.FLOAT, 1, 1, h, w, 16
+        d.window_h = d.window_w = win
+        d.pad_h = d.pad_w = pad
+        d.stride_h = d.stride_w = stride
+        d.global_pooling, d.floor_as_conv = 0, int(floor)
+        oh, ow = C.c_int32(), C.c_int32()
+        assert lib.b200_pool_out_hw(C.byref(d), C.byref(oh), C.byref(ow)) == A.SUCCESS
+        assert (oh.value, ow.value) == want, (h, w, win, pad, stride, floor)
+    wants = reference.value("pool_out_size global sweep", lambda: [
+        oracle.ref_pool_out_size(h, w, 3, 3, 0, 0, 1, 1, True) for h, w in sizes])
+    for (h, w), want in zip(sizes, wants):
+        assert oracle.pool_out_size(h, w, 3, 3, 0, 0, 1, 1, True) == tuple(want)
 
 
 @pytest.mark.parametrize("conv_bias", [False, True])
 @pytest.mark.parametrize("scale_bias", [False, True])
 @pytest.mark.parametrize("factor", [1.0, 0.0, 0.999])
-def test_bn_fold_matches_reference_update_weights(oracle, conv_bias, scale_bias, factor):
+def test_bn_fold_matches_reference_update_weights(oracle, reference, conv_bias, scale_bias, factor):
     """oracle_fold_bn_scale vs the reference's WeightsFusion<float,X86>::update_weights compiled from
     framework/utils/parameter_fusion.cpp:86-131 (oracle/_ref): bit-exact folded weights and bias."""
     rng = np.random.default_rng(int(conv_bias) * 4 + int(scale_bias) * 2 + int(factor * 10))
@@ -168,12 +205,10 @@ def test_bn_fold_matches_reference_update_weights(oracle, conv_bias, scale_bias,
     var = rng.uniform(0.5, 1.5, k).astype(np.float32)
     gamma = rng.uniform(0.8, 1.2, k).astype(np.float32)
     beta = rng.uniform(-0.1, 0.1, k).astype(np.float32) if scale_bias else None
-    want = oracle.ref_fold_bn_scale(w, b, factor, 1e-5, mean, var, gamma, beta)
-    if want is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     got = oracle.fold_bn_scale(w, b, factor, 1e-5, mean, var, gamma, beta)
-    np.testing.assert_array_equal(got[0], want[0])
-    np.testing.assert_array_equal(got[1], want[1])
+    for i, what in enumerate(("weights", "bias")):
+        reference.assert_equal("bn_fold %s%r" % (what, (conv_bias, scale_bias, factor)), got[i],
+                               lambda: oracle.ref_fold_bn_scale(w, b, factor, 1e-5, mean, var, gamma, beta)[i])
 
 
 # (input unsigned, output dtype, relu): the dtype pairs GemmX8S8S32XConv::dispatch accepts (gemm_x8s8s32x_conv.cpp:287-306);
@@ -184,7 +219,7 @@ _GEMM_CONV_DTYPES = [(True, 7, True), (True, 1, False), (True, 1, True), (False,
 
 @pytest.mark.parametrize("xu,odt,relu", _GEMM_CONV_DTYPES)
 @pytest.mark.parametrize("k,pad,stride,dil", [(1, 0, 1, 1), (3, 1, 1, 1), (3, 1, 2, 1), (3, 0, 1, 1), (1, 0, 2, 1), (3, 2, 1, 2)])
-def test_x86_int8_conv_matches_reference_gemm_conv(oracle, xu, odt, relu, k, pad, stride, dil):
+def test_x86_int8_conv_matches_reference_gemm_conv(oracle, reference, xu, odt, relu, k, pad, stride, dil):
     """The INT8 pipeline the CUDA path is held to -- per-channel weight quantisation, bias pre-scaling, the
     input/output dtype scale table, integer accumulation, (acc + bias) * scale, relu, round-to-nearest-even -- against
     the reference's own x86 INT8 convolution GemmX8S8S32XConv run verbatim (oracle/_ref; only MKL's integer GEMM is a
@@ -196,37 +231,34 @@ def test_x86_int8_conv_matches_reference_gemm_conv(oracle, xu, odt, relu, k, pad
         bias = rng.uniform(-0.5, 0.5, cout).astype(np.float32) if with_bias else None
         in_scale = 0.0173
         kw = dict(stride=(stride, stride), pad=(pad, pad), dil=(dil, dil))
+        case = "gemm_conv%r" % ((xu, odt, relu, k, pad, stride, dil, n, hw, cin, cout, with_bias),)
         # an output scale under which nothing leaves the 8-bit range (the reference's cast does not saturate)
-        yf = oracle.ref_gemm_conv_int8(x, w, bias, in_scale, 1, 1.0, relu=relu, **kw)
-        if yf is None:
-            pytest.skip("oracle/_ref not built (no /root/reference here)")
-        out_scale = float(np.abs(yf).max()) / 120.0 + 1e-6
-        want = oracle.ref_gemm_conv_int8(x, w, bias, in_scale, odt, out_scale, relu=relu, **kw)
+        out_scale = reference.value(case + " out_scale", lambda: float(np.abs(
+            oracle.ref_gemm_conv_int8(x, w, bias, in_scale, 1, 1.0, relu=relu, **kw)).max()) / 120.0 + 1e-6)
         wq, ws = oracle.quant_weights_per_oc(w)
         sc, bf, _ = oracle.int8_conv_scales(ws, bias, in_scale, 7 if xu else 3, out_scale, odt)
         got = oracle.conv_s8_nhwc_x86(x, wq, bf if with_bias else None, sc, out_dtype=odt, relu=relu, **kw)
-        np.testing.assert_array_equal(got, want)
+        reference.assert_equal(case, got, lambda: oracle.ref_gemm_conv_int8(x, w, bias, in_scale, odt, out_scale,
+                                                                             relu=relu, **kw))
 
 
-def test_int8_quantisation_helpers_match_reference_scale_utils(oracle):
+def test_int8_quantisation_helpers_match_reference_scale_utils(oracle, reference):
     """The x86 INT8 quantisation rules restated in oracle.c vs the reference's own utils::ScaleUtils
     (saber/funcs/impl/x86/x86_utils.h:293-372) compiled into oracle/_ref: per-output-channel weight quantisation
     (truncating cast), activation quantisation to s8 (roundf + clamp) and to u8 (scale * 127/255, truncation)."""
     rng = np.random.default_rng(11)
     w = (rng.standard_normal((48, 20, 3, 3)) * rng.uniform(0.01, 3.0, (48, 1, 1, 1))).astype(np.float32)
-    want = oracle.ref_quant_weights_per_oc(w)
-    if want is None:
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
     got = oracle.quant_weights_per_oc(w)
-    np.testing.assert_array_equal(got[0], want[0])
-    np.testing.assert_array_equal(got[1], want[1])
+    for i, what in enumerate(("weights", "scales")):
+        reference.assert_equal("quant_weights_per_oc " + what, got[i], lambda: oracle.ref_quant_weights_per_oc(w)[i])
     x = np.concatenate([rng.uniform(-3, 3, 5000), [0.5, -0.5, 1.5, -1.5, 2.5, 126.5, 127.5, -128.5, 3e4, -3e4]]).astype(np.float32)
     for scale in (0.013, 0.02362, 1.0):
-        np.testing.assert_array_equal(oracle.quant_fp32_s8(x * scale, scale), oracle.ref_quant_fp32(x * scale, scale))
+        reference.assert_equal("quant_fp32_s8 scale=%r" % scale, oracle.quant_fp32_s8(x * scale, scale),
+                               lambda: oracle.ref_quant_fp32(x * scale, scale))
     xu = np.concatenate([rng.uniform(0, 3, 5000), [0.0, 0.999, 1.0, 254.9, 255.0]]).astype(np.float32)
     for scale in (0.013, 0.02362):
-        np.testing.assert_array_equal(oracle.quant_fp32_u8(xu * scale * 127 / 255, scale),
-                                      oracle.ref_quant_fp32(xu * scale * 127 / 255, scale, unsigned=True))
+        reference.assert_equal("quant_fp32_u8 scale=%r" % scale, oracle.quant_fp32_u8(xu * scale * 127 / 255, scale),
+                               lambda: oracle.ref_quant_fp32(xu * scale * 127 / 255, scale, unsigned=True))
 
 
 def test_bn_fold_equals_unfused_ops(oracle):
@@ -316,53 +348,55 @@ def test_softmax_eltwise_activation_oracles(oracle):
 @pytest.mark.parametrize("ptype", [1, 2, 3])            # max, avg incl. padding, avg excl. padding
 @pytest.mark.parametrize("window,pad,stride", [((2, 2), (0, 0), (2, 2)), ((3, 3), (1, 1), (2, 2)), ((3, 3), (0, 0), (2, 2)),
                                                ((3, 2), (1, 0), (1, 2)), ((2, 2), (1, 1), (1, 1)), ((7, 7), (0, 0), (1, 1))])
-def test_pool_f32_matches_reference_test_oracle(oracle, ptype, window, pad, stride):
+def test_pool_f32_matches_reference_test_oracle(oracle, reference, ptype, window, pad, stride):
     rng = np.random.default_rng(hash((ptype, window, pad, stride)) % 2 ** 31)
     for shape in [(1, 3, 7, 7), (2, 4, 12, 21), (3, 2, 24, 24)]:
         x = rng.uniform(-1, 1, shape).astype(np.float32)
-        np.testing.assert_array_equal(oracle.pool_f32(x, window, pad, stride, ptype),
-                                      oracle.ref_pool_f32(x, window, pad, stride, ptype))
+        reference.assert_equal("pool_f32%r" % ((ptype, window, pad, stride, shape),),
+                               oracle.pool_f32(x, window, pad, stride, ptype),
+                               lambda: oracle.ref_pool_f32(x, window, pad, stride, ptype))
 
 
 @pytest.mark.parametrize("m,k,n", [(1, 16, 4), (3, 100, 37), (8, 2048, 1000), (2, 25088, 16)])
 @pytest.mark.parametrize("bias", [False, True])
-def test_fc_f32_matches_reference_test_oracle(oracle, m, k, n, bias):
+def test_fc_f32_matches_reference_test_oracle(oracle, reference, m, k, n, bias):
     rng = np.random.default_rng(m * 131 + k + n)
     x = rng.uniform(-1, 1, (m, k)).astype(np.float32)
     w = rng.uniform(-1, 1, (n, k)).astype(np.float32)
     b = rng.uniform(-1, 1, n).astype(np.float32) if bias else None
-    np.testing.assert_array_equal(oracle.fc_f32(x, w, b), oracle.ref_fc_f32(x, w, b))
+    reference.assert_equal("fc_f32%r" % ((m, k, n, bias),), oracle.fc_f32(x, w, b), lambda: oracle.ref_fc_f32(x, w, b))
 
 
 @pytest.mark.parametrize("shape", [(1, 1000, 1, 1), (8, 1000, 1, 1), (2, 5, 3, 4), (3, 21, 7, 2)])
 @pytest.mark.parametrize("axis", [1, 2, 3])
-def test_softmax_matches_reference_test_oracle(oracle, shape, axis):
+def test_softmax_matches_reference_test_oracle(oracle, reference, shape, axis):
     rng = np.random.default_rng(sum(shape) + axis)
     x = rng.uniform(-6, 6, shape).astype(np.float32)
     outer, inner = int(np.prod(shape[:axis])), int(np.prod(shape[axis + 1:]))
-    np.testing.assert_array_equal(oracle.softmax_f32(x, outer, shape[axis], inner), oracle.ref_softmax_f32(x, axis))
+    reference.assert_equal("softmax%r" % ((shape, axis),), oracle.softmax_f32(x, outer, shape[axis], inner),
+                           lambda: oracle.ref_softmax_f32(x, axis))
 
 
 @pytest.mark.parametrize("op,coeff", [(2, (1.0, 1.0)), (2, (0.5, -1.5)), (1, (1.0, 1.0)), (3, (1.0, 1.0))])   # sum, prod, max
 @pytest.mark.parametrize("relu", [False, True])
-def test_eltwise_matches_reference_test_oracle(oracle, op, coeff, relu):
+def test_eltwise_matches_reference_test_oracle(oracle, reference, op, coeff, relu):
     rng = np.random.default_rng(op * 7 + int(relu))
     a = rng.uniform(-2, 2, 4099).astype(np.float32)
     b = rng.uniform(-2, 2, 4099).astype(np.float32)
-    np.testing.assert_array_equal(oracle.eltwise_f32(a, b, op, coeff[0], coeff[1], relu),
-                                  oracle.ref_eltwise_f32(a, b, op, coeff[0], coeff[1], relu))
+    reference.assert_equal("eltwise%r" % ((op, coeff, relu),), oracle.eltwise_f32(a, b, op, coeff[0], coeff[1], relu),
+                           lambda: oracle.ref_eltwise_f32(a, b, op, coeff[0], coeff[1], relu))
 
 
 @pytest.mark.parametrize("act,coef", [(2, 1.0), (1, 1.0), (3, 1.0), (4, 1.5), (5, 0.7)])   # relu sigmoid tanh clipped elu
-def test_activation_matches_reference_test_oracle(oracle, act, coef):
+def test_activation_matches_reference_test_oracle(oracle, reference, act, coef):
     x = np.random.default_rng(act).uniform(-4, 4, (2, 3, 5, 7)).astype(np.float32)
-    np.testing.assert_array_equal(oracle.activation_f32(x, act, 0.0, coef), oracle.ref_activation_f32(x, act, 0.0, coef))
+    reference.assert_equal("activation%r" % ((act, coef),), oracle.activation_f32(x, act, 0.0, coef),
+                           lambda: oracle.ref_activation_f32(x, act, 0.0, coef))
 
 
-def test_grouped_x86_int8_conv_agrees_with_reference_oracle_on_shared_subset(oracle):
+def test_grouped_x86_int8_conv_agrees_with_reference_oracle_on_shared_subset(oracle, reference):
     """Depthwise / grouped INT8: the grouped x86 restatement coincides with the reference's own conv_basic_check_int8
     (which takes `group`) on their shared subset -- integral bias, s8 output, no residual."""
-    _need_ref(oracle)
     rng = np.random.default_rng(23)
     for c, k, group in ((16, 16, 16), (32, 32, 32), (16, 32, 4)):
         x = rng.integers(-128, 128, (2, 9, 9, c)).astype(np.int8)
@@ -370,10 +404,11 @@ def test_grouped_x86_int8_conv_agrees_with_reference_oracle_on_shared_subset(ora
         b = rng.integers(-1000, 1000, k).astype(np.int32)
         sc = rng.uniform(0.002, 0.02, k).astype(np.float32)
         for relu in (False, True):
-            r = oracle.conv_s8_nhwc_basic(x, w, b, sc, pad=(1, 1), stride=(2, 2), relu=relu, group=group, use_ref=True)
             j = oracle.conv_s8_nhwc_x86(x, w, b.astype(np.float32), sc, pad=(1, 1), stride=(2, 2), relu=relu,
                                         out_dtype=oracle.DT_INT8, group=group)
-            np.testing.assert_array_equal(j, r)
+            reference.assert_equal("conv_int8_basic grouped%r" % ((c, k, group, relu),), j,
+                                   lambda: oracle.conv_s8_nhwc_basic(x, w, b, sc, pad=(1, 1), stride=(2, 2), relu=relu,
+                                                                     group=group, use_ref=True))
     # group == 1 through the grouped entry point is the ungrouped function
     x = rng.integers(0, 256, (1, 7, 7, 16)).astype(np.uint8)
     w = rng.integers(-127, 128, (8, 16, 3, 3)).astype(np.int8)
